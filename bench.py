@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                (N > 1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   (the reference's CPU path: oracle C port, all host threads)
     python bench.py --soak 60 --gpus N                            (BASELINE configs[4]: sustained mixed ingest, own JSON line)
+    python bench.py --steps K --dump-outputs DIR                  (also writes the last timed step's result bitmap as DIR/verify_ok.npy)
 
 A "step" is one pass of the hot path over one batch: per GPU, configs[1] of BASELINE.json — batched Ed25519 verify of
 1 M x 512 B credentials (K = 1024 key pairs, 1 % corrupted so the kernel cannot short-circuit; SURVEY.md §8d).  Weak
@@ -36,6 +37,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree untouched (it may be read-only); only --dump-outputs writes
 
 N_ITEMS = 1_000_000
 MSG_LEN = 512
@@ -342,6 +344,14 @@ def timed_loop(fn, steps, barrier):
     return e0.elapsed_time(e1)
 
 
+def dump_outputs(out_dir, arrays):
+    """Write device tensors as out_dir/<name>.npy in float32.  The inputs are seeded, so the files of two builds run with the same
+    arguments can be compared item by item."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
 def cfg4_block(ctx, dev, rank, world, barrier, reps=3):
     """BASELINE configs[3]: 2^22 sign + RFC 6962 append over the ranks, NCCL all-gather of the subtree roots, fold; timed on the
     device (max over ranks), then checked against a single-rank recomputation of the whole log on rank 0."""
@@ -500,7 +510,12 @@ def main():
     ap.add_argument("--soak", type=float, default=0.0, help="BASELINE configs[4]: sustained mixed ingest for this many seconds (own JSON line)")
     ap.add_argument("--soak-rate", type=float, default=100_000.0, help="whole-job target rate of --soak, actions/s")
     ap.add_argument("--extras", action="store_true", help="also time sign / canonical form / microbenchmarks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (the 1 M-entry verify bitmap, 4 MB) as DIR/verify_ok.npy "
+                         "in float32; rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -590,6 +605,8 @@ def main():
     launches = ctx.launch_count() - launches0
     clocks = sampler.stop()
     assert torch.equal(d_ok, expect)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"verify_ok": d_ok})
     t_ms = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)

@@ -60,9 +60,11 @@ def test_product_never_imports_or_links_the_oracle():
 
 
 def test_kernels_are_sm100a_sass():
+    import shutil
     import subprocess
     so = os.path.join(ROOT, "agentfield_b200", "libafcrypto.so")
-    out = subprocess.check_output(["cuobjdump", "-lelf", so]).decode()
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
+    out = subprocess.check_output([cuobjdump, "-lelf", so]).decode()
     assert "sm_100a" in out and "sm_90" not in out and "sm_80" not in out
 
 
